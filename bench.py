@@ -12,13 +12,17 @@ Multi-GPU: one process per GPU (torchrun), voices sharded contiguously (weak sca
 stereo/mono partial mixes are summed with one NCCL reduce per step (SURVEY.md §8e).
 """
 import argparse
+import atexit
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
+sys.dont_write_bytecode = True   # the tree may be read-only: no __pycache__ from the modules imported below
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "tests")):
     if p not in sys.path:
@@ -47,7 +51,64 @@ def parse():
     ap.add_argument("--seconds", type=float, default=1.0, help="audio seconds rendered per step")
     ap.add_argument("--per-voice", action="store_true", help="also materialise per-voice outputs in HBM (value only)")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"], help="weak: --voices per GPU (default); strong: the config's voices split over the GPUs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last timed step as DIR/<name>.npy (float32, at most 64 MB in all); "
+                         "the warm-up is then exactly max(3, --warmup) steps, so the same arguments give the same outputs")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_sample(shape, budget, itemsize=4):
+    """Row and column indices of a [rows, cols] output that fit in `budget` bytes: all of it when it fits, else a fixed, seeded sample
+    of rows (and, if one row alone is too large, of columns), the same for the same shape so that two builds dump the same elements."""
+    import numpy as np
+    rows, cols = shape
+    rng = np.random.default_rng(0)
+    r, c = np.arange(rows), np.arange(cols)
+    if rows * cols * itemsize > budget:
+        r = np.sort(rng.choice(rows, min(rows, max(1, budget // (cols * itemsize))), replace=False))
+    if len(r) * cols * itemsize > budget:
+        c = np.sort(rng.choice(cols, max(1, budget // (len(r) * itemsize)), replace=False))
+    return r, c
+
+
+def dump_outputs(d, arrays):
+    """`arrays`: {name: callable(rows, cols) -> float32 ndarray of those rows and columns, shape}; each gets an equal share of DUMP_BYTES."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    for name, (take, shape) in arrays.items():
+        r, c = dump_sample(shape, DUMP_BYTES // len(arrays))
+        np.save(os.path.join(d, name + ".npy"), np.ascontiguousarray(take(r, c), dtype=np.float32))
+
+
+_SCRATCH = []
+
+
+def scratch_dir():
+    """What the run compiles or caches goes here, never into the tree (which may be read-only); removed at exit."""
+    if not _SCRATCH:
+        _SCRATCH.append(tempfile.mkdtemp(prefix="fundsp_bench_"))
+        atexit.register(shutil.rmtree, _SCRATCH[0], True)
+    return _SCRATCH[0]
+
+
+def jit_cache_overlay():
+    """Points the JIT disk cache at a scratch directory holding links to the units build() compiled into fundsp_b200/jit_cache: those
+    are still hits, and a unit compiled during the run is stored beside them instead of in the tree. An explicit FDSP_JIT_CACHE wins."""
+    if os.environ.get("FDSP_JIT_CACHE"):
+        return
+    d = os.path.join(scratch_dir(), "jit_cache")
+    os.makedirs(d)
+    src = os.path.join(ROOT, "fundsp_b200", "jit_cache")
+    for f in (os.listdir(src) if os.path.isdir(src) else ()):
+        if f.endswith(".fdspjit"):
+            os.symlink(os.path.join(src, f), os.path.join(d, f))
+    os.environ["FDSP_JIT_CACHE"] = d
 
 
 class ClockSampler:
@@ -109,10 +170,10 @@ def host_cores():
 
 def native_oracle():
     """The timed CPU arm runs the oracle built for THIS host (-march=native, as BASELINE.md §3 states); the parity tests keep the
-    portable x86-64-v3 build. Built once per box next to the portable one; falls back to it if the compiler is missing."""
-    so = os.path.join(ROOT, "oracle", "_build", "libfundsp_oracle_native.so")
+    portable x86-64-v3 build. Built per run in the scratch directory; falls back to the portable build if the compiler is missing."""
+    so = os.path.join(scratch_dir(), "libfundsp_oracle_native.so")
     try:
-        subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "native"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL, timeout=600)
+        subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "native", "NATIVE=" + so], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL, timeout=600)
         if os.path.exists(so):
             os.environ["FDSP_ORACLE_SO"] = so
             return "g++ -O3 -march=native -ffp-contract=off"
@@ -155,8 +216,10 @@ def run_reference(a):
         cpu_reference(a.workload, V, min(ns, 4800), cores)
     ts = []
     for _ in range(a.steps):
-        dt, _ = cpu_reference(a.workload, V, ns, cores)
+        dt, mix = cpu_reference(a.workload, V, ns, cores)
         ts.append(dt)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"mix": (lambda r, c: mix[r][:, c], mix.shape)})
     t = sum(ts) / len(ts)
     val = V * ns / t / 1e6
     v1 = min(V, 64)
@@ -211,6 +274,7 @@ def main():
     rank, world, local = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1")), int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device; fundsp_b200 has no CPU fallback (use --impl reference for the CPU arm)")
+    jit_cache_overlay()
     torch.cuda.set_device(local)
     dist = None
     group = None
@@ -295,7 +359,8 @@ def main():
         device_step()
         e2e_step()
     per = (time.perf_counter() - t_w) / max(3, a.warmup)
-    extra = torch.tensor([min(500, max(0, int(1.0 / max(per, 1e-4))))], device="cuda", dtype=torch.int64)
+    # (with --dump-outputs no extra steps: their number depends on timing, and every step advances the bank's state)
+    extra = torch.tensor([0 if a.dump_outputs else min(500, max(0, int(1.0 / max(per, 1e-4))))], device="cuda", dtype=torch.int64)
     if dist is not None:
         dist.broadcast(extra, src=0)
     for _ in range(int(extra.item())):
@@ -307,6 +372,10 @@ def main():
     if not ms_dom > 0.0:            # FDSP_NO_DOM=1 (the A/B switch of those event records): fall back on the whole device region
         ms_dom = ms_kernel
     launches = bank.launch_count() - launches0
+    if a.dump_outputs and rank == 0:   # the mix (reduced over the ranks) and, with --per-voice, this rank's voice rows
+        def take(t):
+            return lambda r, c: t[torch.from_numpy(r).cuda()][:, torch.from_numpy(c).cuda()].cpu().numpy()
+        dump_outputs(a.dump_outputs, {"mix": (take(mix), tuple(mix.shape)), **({"voices": (take(out), tuple(out.shape))} if out is not None else {})})
     ms_e2e, _, _ = timed(e2e_step, a.steps)
     # AudioUnit::process granularity: one C-ABI call per 64-sample block with host buffers (the Wave::render call pattern)
     pb = 200

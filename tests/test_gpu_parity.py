@@ -417,7 +417,7 @@ def test_fdn_kernel_process_granularity_and_wet_only_pipe():
         assert np.abs(g - ref).max() <= 1e-5 * max(1.0, np.abs(per_voice).sum(axis=0).max())
 
 
-def test_fdn_kernel_equals_generic_thread_per_voice_form():
+def test_fdn_kernel_equals_generic_thread_per_voice_form(tmp_path):
     """The specialised kernel and the generic lowering of the same graph must agree bit for bit."""
     import os
     import subprocess
@@ -427,7 +427,7 @@ def test_fdn_kernel_equals_generic_thread_per_voice_form():
             "np.save(sys.argv[1], g); print(b.classes()[0]['signature'][:20])")
     outs = []
     for k, env in enumerate(({}, {"FDSP_DISABLE_FDN": "1"})):
-        path = f"/tmp/fdn_ab_{k}.npy"
+        path = str(tmp_path / f"fdn_ab_{k}.npy")
         subprocess.check_call([sys.executable, "-c", code, path], env={**os.environ, **env}, cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
         outs.append(np.load(path))
     assert np.array_equal(outs[0], outs[1]) and np.abs(outs[0]).max() > 0.01
