@@ -27,6 +27,24 @@ struct WaveTableDev {
 FDSP_HDC constexpr int mix_tile_samples(int outs) { return outs <= 1 ? 64 : (outs == 2 ? 32 : (outs <= 4 ? 16 : 8)); }
 FDSP_HDC constexpr size_t mix_tile_floats(int outs, int nt) { return (size_t)outs * (size_t)mix_tile_samples(outs) * (size_t)(nt + 1); }
 
+// Hand-off rings of the stage-pipelined kernel (bank_kernel_st.cuh): per channel crossing a stage boundary and voice slot of the CTA,
+// ST_NSLOT slots of HS samples.
+constexpr int ST_NSLOT = 2;
+FDSP_HDC constexpr int st_hand_samples(int outs, bool mix) { return mix && mix_tile_samples(outs) < 16 ? mix_tile_samples(outs) : 16; }
+FDSP_HDC constexpr size_t st_ring_floats(int outs, int mid_sum, int nt, bool mix) { return (size_t)ST_NSLOT * mid_sum * st_hand_samples(outs, mix) * nt; }
+
+// Dynamic shared memory of a bank launch of nt voices per CTA: the mix tile (mode bit 1), the hand-off rings when the launch is
+// stage-pipelined (mid_sum channels cross its stage boundaries; 0 otherwise), then the wavetables (table_bytes; 0 when the class reads
+// none), which are staged (tb) only when all of it fits in the shared memory a block may have.
+constexpr size_t SMEM_BLOCK_MAX = 227 * 1024;
+struct LaunchSmem { bool tb; size_t smem; };
+FDSP_HDC inline LaunchSmem launch_smem(int outs, int nt, int mid_sum, int mode, size_t table_bytes) {
+  const bool mix = (mode & 2) != 0;
+  const size_t base = (mix ? sizeof(float) * mix_tile_floats(outs, nt) : 0) + sizeof(float) * st_ring_floats(outs, mid_sum, nt, mix);
+  const bool tb = table_bytes > 0 && base + table_bytes <= SMEM_BLOCK_MAX;
+  return {tb, base + (tb ? table_bytes : 0)};
+}
+
 // CTA shape of a class of V voices with NT threads per CTA: enough CTAs to cover the voices, rounded up to whole waves of the
 // 148 SMs once every CTA can still have a full warp, and the voices spread evenly over them (a bank is bound by per-SM
 // pipes and per-warp latency, so idle SMs are the first thing to use up).

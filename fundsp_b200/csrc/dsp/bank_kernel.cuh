@@ -10,7 +10,8 @@
 // column sums), finished by mix_reduce_kernel in CTA order (deterministic).
 #pragma once
 #include "nodes.cuh"
-#include "bank_args.h"
+#include "mix_order.h"
+#include "voice_block.cuh"
 
 namespace fdsp {
 
@@ -36,16 +37,22 @@ FDSP_DEV void mbar_wait(uint32_t bar, uint32_t parity) {
       : "memory");
 }
 
-// TB: stage the wavetable data of kind WaveKind<G> in shared memory behind the mix tile (one TMA bulk copy per
-// 32 KB slice, single mbarrier), so the per-sample table taps become conflict-light LDS instead of divergent LDG.
+// TB: stage the wavetable data of kind WaveKind<G> in shared memory at `tsm` (one TMA bulk copy per 32 KB slice on the initialised
+// mbarrier `bar`), so the per-sample table taps become conflict-light LDS instead of divergent LDG; then point the context at it.
+template <class G, class C> FDSP_DEV void stage_tables(const BankArgs& a, float* tsm, uint32_t bar, C& c) {
+  constexpr int KIND = WaveKind<G>::value >= 0 ? WaveKind<G>::value : 0;
+  const uint32_t bytes = (uint32_t)a.wt[KIND].total * 4u;
+  if (threadIdx.x == 0) {
+    mbar_expect_tx(bar, bytes);
+    const char* src = reinterpret_cast<const char*>(a.wt[KIND].data);
+    for (uint32_t o = 0; o < bytes; o += 32768u) bulk_g2s(smem_addr(tsm) + o, src + o, (bytes - o) < 32768u ? (bytes - o) : 32768u, bar);
+  }
+  mbar_wait(bar, 0);
+  c.tsm = smem_addr(tsm); c.tsm_kind = KIND;
+}
+
 #ifndef FDSP_MIN_CTAS
 #define FDSP_MIN_CTAS 1   // one resident CTA per SM is all a bank needs: lets ptxas spend registers on overlapping the 8-sample group
-#endif
-#ifndef FDSP_NO_GROUP
-#define FDSP_NO_GROUP 0
-#endif
-#ifndef FDSP_GROUP_COST
-#define FDSP_GROUP_COST 256   // programs whose group form unrolls to at most this many instructions per sample are evaluated 8 samples at a time
 #endif
 
 template <class G, int NT, int MODE, bool TB>
@@ -57,31 +64,16 @@ __global__ void __launch_bounds__(NT, FDSP_MIN_CTAS) bank_kernel(const BankArgs 
   const bool active = tid < vpc && v < a.V;
   constexpr int IN = G::IN, OUT = G::OUT;
   constexpr int TS = (MODE & 2) ? mix_tile_samples(OUT) : 64;
-  // big programs (e.g. the 32-line FDN in thread-per-voice form) are not unrolled over the 8-sample group
-  constexpr bool GROUP = GroupPlan<G>::ok && GroupPlan<G>::code <= FDSP_GROUP_COST && !FDSP_NO_GROUP;
-  constexpr int UNROLL = GROUP ? 8 : (Cost<G>::value <= 160 ? 8 : (Cost<G>::value <= 320 ? 4 : (Cost<G>::value <= 640 ? 2 : 1)));
 
   typename G::R r;
-  CtxT<TB> c;
-  c.tsm = 0u; c.tsm_kind = -1;
+  CtxT<TB> c = voice_ctx<TB>(a, v);
   if (TB) {
-    constexpr int KIND = WaveKind<G>::value >= 0 ? WaveKind<G>::value : 0;
     __shared__ __align__(8) unsigned long long mbar;
-    float* tsm = tile + ((MODE & 2) ? mix_tile_floats(OUT, NT) : 0);
-    const uint32_t bytes = (uint32_t)a.wt[KIND].total * 4u;
     const uint32_t bar = smem_addr(&mbar);
     if (tid == 0) mbar_init(bar, 1);
     __syncthreads();
-    if (tid == 0) {
-      mbar_expect_tx(bar, bytes);
-      const char* src = reinterpret_cast<const char*>(a.wt[KIND].data);
-      for (uint32_t o = 0; o < bytes; o += 32768u) bulk_g2s(smem_addr(tsm) + o, src + o, (bytes - o) < 32768u ? (bytes - o) : 32768u, bar);
-    }
-    mbar_wait(bar, 0);
-    c.tsm = smem_addr(tsm); c.tsm_kind = KIND;
+    stage_tables<G>(a, tile + ((MODE & 2) ? mix_tile_floats(OUT, NT) : 0), bar, c);
   }
-  c.wt = a.wt; c.dl = a.dline; c.V = a.V; c.v = v; c.sr = a.sr; c.sd64 = a.sd64; c.sd32 = a.sd32;
-  c.rp = a.params; c.rs0 = a.state0; c.ru = a.uniform; c.dl_total = a.dl_floats;
   if (active) {
     Loader l{a.params, a.state, a.uniform, a.V, v, 0u, 0u, 0u, 0u};
     G::load(r, l);
@@ -93,102 +85,45 @@ __global__ void __launch_bounds__(NT, FDSP_MIN_CTAS) bank_kernel(const BankArgs 
 #pragma unroll 1
   for (uint32_t t0 = 0; t0 < a.n; t0 += 64) {
     const int nb = (a.n - t0) < 64u ? (int)(a.n - t0) : 64;
-    const int nfull = nb & ~7;
-    c.n = nb;
     float* orow = (active && (MODE & 1)) ? a.out + (size_t)__ldg(a.row_map + v) * a.out_stride + a.out_offset + t0 : nullptr;
     const float* irow = (IN > 0) ? a.in + a.in_offset + t0 : nullptr;
 #pragma unroll 1
     for (int s0 = 0; s0 < nb; s0 += TS) {   // one pass when there is no mix tile (TS = 64)
       const int s1 = (s0 + TS) < nb ? (s0 + TS) : nb;
       if (active) {
-        const int gend = s1 < nfull ? s1 : nfull;
-        c.rem = false;
-#pragma unroll 1
-        for (int g = s0; g < gend; g += 8) {
-          float ob[OUT > 0 ? OUT : 1][8];
-          if constexpr (GROUP) {
-            // small programs: node by node over the 8-sample group (group_step), all intermediates in registers
-            Fr8<IN> in8; Fr8<OUT> o8;
+        walk_block<G>(
+            r, c, nb, s0, s1, [&](int k, int i, int j) { return __ldg(irow + (size_t)k * a.in_stride + i + j); },
+            [&](int k, int i, float y) {
+              if (MODE & 2) tile[(k * TS + (i - s0)) * (NT + 1) + tid] = y;
+            },
+            [&](int k, int g, const float (&y)[8]) {
+              if (MODE & 1) {
+                float* p = orow + (size_t)k * a.out_stride + g;
+                if (vec_ok) {
+                  *reinterpret_cast<float4*>(p) = make_float4(y[0], y[1], y[2], y[3]);
+                  *reinterpret_cast<float4*>(p + 4) = make_float4(y[4], y[5], y[6], y[7]);
+                } else {
 #pragma unroll
-            for (int k = 0; k < IN; k++) {
-#pragma unroll
-              for (int j = 0; j < 8; j++) in8.v[k][j] = __ldg(irow + (size_t)k * a.in_stride + g + j);
-            }
-            c.i = g; c.first = true;
-            group_step<G>(r, c, in8, o8);
-#pragma unroll
-            for (int k = 0; k < OUT; k++) {
-#pragma unroll
-              for (int j = 0; j < 8; j++) {
-                ob[k][j] = o8.v[k][j];
-                if (MODE & 2) tile[(k * TS + (g - s0) + j) * (NT + 1) + tid] = o8.v[k][j];
+                  for (int j = 0; j < 8; j++) p[j] = y[j];
+                }
               }
-            }
-          } else {
-#pragma unroll(UNROLL)
-            for (int j = 0; j < 8; j++) {
-              Fr<IN> in; Fr<OUT> o;
-#pragma unroll
-              for (int k = 0; k < IN; k++) in.v[k] = __ldg(irow + (size_t)k * a.in_stride + g + j);
-              c.i = g + j; c.first = (j == 0);
-              G::template step<false>(r, c, in, o);
-#pragma unroll
-              for (int k = 0; k < OUT; k++) {
-                ob[k][j] = o.v[k];
-                if (MODE & 2) tile[(k * TS + (g - s0) + j) * (NT + 1) + tid] = o.v[k];
-              }
-            }
-          }
-          if (MODE & 1) {
-#pragma unroll
-            for (int k = 0; k < OUT; k++) {
-              float* p = orow + (size_t)k * a.out_stride + g;
-              if (vec_ok) {
-                *reinterpret_cast<float4*>(p) = make_float4(ob[k][0], ob[k][1], ob[k][2], ob[k][3]);
-                *reinterpret_cast<float4*>(p + 4) = make_float4(ob[k][4], ob[k][5], ob[k][6], ob[k][7]);
-              } else {
-#pragma unroll
-                for (int j = 0; j < 8; j++) p[j] = ob[k][j];
-              }
-            }
-          }
-        }
-        if (s1 == nb) {  // end of the block: wrap up the SIMD part, then the (size & 7) tail through the tick path
-          G::end_simd(r);
-          c.rem = true; c.first = false;
-#pragma unroll 1
-          for (int i = nfull; i < nb; i++) {
-            Fr<IN> in; Fr<OUT> o;
-#pragma unroll
-            for (int k = 0; k < IN; k++) in.v[k] = __ldg(irow + (size_t)k * a.in_stride + i);
-            c.i = i;
-            G::template step<false>(r, c, in, o);
-#pragma unroll
-            for (int k = 0; k < OUT; k++) {
-              if (MODE & 1) orow[(size_t)k * a.out_stride + i] = o.v[k];
-              if (MODE & 2) tile[(k * TS + (i - s0)) * (NT + 1) + tid] = o.v[k];
-            }
-          }
-        }
+            },
+            [&](int k, int i, float y) {
+              if (MODE & 1) orow[(size_t)k * a.out_stride + i] = y;
+              if (MODE & 2) tile[(k * TS + (i - s0)) * (NT + 1) + tid] = y;
+            });
       }
       if (MODE & 2) {
-        // CTA partial mix: two threads per (channel, sample) row, each folding one half of the voice columns with four
-        // interleaved accumulators; fixed association ((a0+a1)+(a2+a3)) then low half + high half -> deterministic.
+        // CTA partial mix: two threads per (channel, sample) row, each folding one half of the voice columns (mix_order.h)
         __syncthreads();
-        constexpr int HALF = NT / 2, QN = HALF / 4, ROWS = OUT * TS;
+        constexpr int HALF = NT / 2, ROWS = OUT * TS;
         const int h = (int)(tid & 1u);
-        // the odd thread starts QN columns further so that the 32 lanes of a warp (16 rows x 2 halves) hit 32 banks
-        const int c0 = h * HALF + (h * QN) % HALF, c1 = h * HALF + (QN + h * QN) % HALF, c2 = h * HALF + (2 * QN + h * QN) % HALF, c3 = h * HALF + (3 * QN + h * QN) % HALF;
 #pragma unroll 1
         for (int eb = (int)(tid >> 5) * 16; eb < ROWS; eb += HALF) {   // warp-uniform trip count (full-mask shuffle below)
           const int e = eb + (int)((tid & 31u) >> 1);
           const bool ok = e < ROWS;
           const int k = e / TS, i = e - k * TS;
-          const float* row = tile + (ok ? e : 0) * (NT + 1);
-          float a0 = row[c0], a1 = row[c1], a2 = row[c2], a3 = row[c3];
-#pragma unroll
-          for (int q = 1; q < QN; q++) { a0 += row[c0 + q]; a1 += row[c1 + q]; a2 += row[c2 + q]; a3 += row[c3 + q]; }
-          const float s = (a0 + a1) + (a2 + a3);
+          const float s = cta_half_row_sum<NT>(tile + (ok ? e : 0) * (NT + 1), h);
           const float other = __shfl_xor_sync(0xffffffffu, s, 1);
           if (ok && h == 0 && s0 + i < s1) a.partial[((size_t)blockIdx.x * OUT + k) * a.n + t0 + s0 + i] = s + other;
         }
@@ -210,8 +145,7 @@ __global__ void __launch_bounds__(NT, FDSP_MIN_CTAS) bank_kernel(const BankArgs 
       __threadfence();
       for (uint32_t e = tid; e < (uint32_t)OUT * a.n; e += NT) {
         const uint32_t ch = e / a.n, t = e - ch * a.n;
-        float s = __ldcg(a.partial + (size_t)ch * a.n + t);
-        for (uint32_t b = 1; b < gridDim.x; b++) s += __ldcg(a.partial + ((size_t)b * OUT + ch) * a.n + t);
+        const float s = cta_order_fold(a.partial + (size_t)ch * a.n + t, (size_t)OUT * a.n, gridDim.x, [](const float* p) { return __ldcg(p); });
         float* p = a.mix + (size_t)ch * a.mix_stride + a.mix_offset + t;
         *p = a.mix_accumulate ? *p + s : s;
       }
@@ -226,8 +160,7 @@ static __global__ void mix_reduce_kernel(const float* partial, uint32_t nparts, 
   const uint32_t e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= outs * n) return;
   const uint32_t c = e / n, t = e % n;
-  float s = partial[(size_t)c * n + t];
-  for (uint32_t b = 1; b < nparts; b++) s += partial[((size_t)b * outs + c) * n + t];
+  const float s = cta_order_fold(partial + (size_t)c * n + t, (size_t)outs * n, nparts, [](const float* p) { return *p; });
   float* p = mix + (size_t)c * mix_stride + mix_offset + t;
   *p = accumulate ? *p + s : s;
 }
@@ -255,11 +188,7 @@ static __global__ void tree_mix_block_kernel(const float* __restrict__ rows, uin
 #pragma unroll
     for (int u = 0; u < 8; u++) b[u] = __ldg(p + (size_t)(v0 + u) * vstep);
 #pragma unroll
-    for (int u = 0; u < 8; u++) {
-      float y = b[u]; uint32_t q = v0 + u; int lvl = 0;
-      while (q & 1u) { y = st[lvl] + y; q >>= 1; lvl++; }
-      st[lvl] = y;
-    }
+    for (int u = 0; u < 8; u++) carry_push(st, b[u], v0 + u, 0);
   }
   partial[((size_t)blk * outs + ch) * n + t] = st[LB];
 }
@@ -277,9 +206,7 @@ static __global__ void tree_mix_kernel(const float* __restrict__ rows, uint32_t 
     float st[32];
     // complete blocks of 2^lb voices arrive as their subtree sums (tree_mix_block_kernel): pushed at level lb with the block index as the carry pattern
     for (uint32_t bk = 0; bk < nfull; bk++) {
-      float y = __ldg(partial + ((size_t)bk * outs + ch) * n + t); uint32_t q = bk; int lvl = lb;
-      while (q & 1u) { y = st[lvl] + y; q >>= 1; lvl++; }
-      st[lvl] = y;
+      carry_push(st, __ldg(partial + ((size_t)bk * outs + ch) * n + t), bk, lb);
     }
     for (uint32_t v0 = nfull << lb; v0 < V; v0 += 8) {
       float b[8];
@@ -287,17 +214,10 @@ static __global__ void tree_mix_kernel(const float* __restrict__ rows, uint32_t 
       for (int u = 0; u < 8; u++) b[u] = (v0 + u < V) ? __ldg(p + (size_t)(v0 + u) * vstep) : 0.0f;
 #pragma unroll
       for (int u = 0; u < 8; u++) {
-        if (v0 + u < V) {
-          float y = b[u]; uint32_t q = v0 + u; int lvl = 0;
-          while (q & 1u) { y = st[lvl] + y; q >>= 1; lvl++; }
-          st[lvl] = y;
-        }
+        if (v0 + u < V) carry_push(st, b[u], v0 + u, 0);
       }
     }
-    int lvl = 0; uint32_t q = V;
-    while (!(q & 1u)) { q >>= 1; lvl++; }
-    x = st[lvl]; q >>= 1; lvl++;
-    for (; q; q >>= 1, lvl++) if (q & 1u) x = st[lvl] + x;
+    x = carry_finish(st, V);
   } else {
     x = __ldg(p);
     for (uint32_t v = 1; v < V; v++) x += __ldg(p + (size_t)v * vstep);

@@ -30,29 +30,15 @@ __global__ void __launch_bounds__(NT, FDSP_MIN_CTAS) bank_kernel_rt(const BankAr
   const bool active = tid < vpc && v < a.V;
   constexpr int IN = G::IN, OUT = G::OUT;
   constexpr int TS = mix_tile_samples(OUT);
-  constexpr bool GROUP = GroupPlan<G>::ok && GroupPlan<G>::code <= FDSP_GROUP_COST && !FDSP_NO_GROUP;
-  constexpr int UNROLL = GROUP ? 8 : (Cost<G>::value <= 160 ? 8 : (Cost<G>::value <= 320 ? 4 : (Cost<G>::value <= 640 ? 2 : 1)));
   typename G::R r;
-  CtxT<TB> c;
-  c.tsm = 0u; c.tsm_kind = -1;
+  CtxT<TB> c = voice_ctx<TB>(a, v);
   if (TB) {
-    constexpr int KIND = WaveKind<G>::value >= 0 ? WaveKind<G>::value : 0;
     __shared__ __align__(8) unsigned long long mbar;
-    float* tsm = tile + mix_tile_floats(OUT, NT);
-    const uint32_t bytes = (uint32_t)a.wt[KIND].total * 4u;
     const uint32_t bar = smem_addr(&mbar);
     if (tid == 0) mbar_init(bar, 1);
     __syncthreads();
-    if (tid == 0) {
-      mbar_expect_tx(bar, bytes);
-      const char* src = reinterpret_cast<const char*>(a.wt[KIND].data);
-      for (uint32_t o = 0; o < bytes; o += 32768u) bulk_g2s(smem_addr(tsm) + o, src + o, (bytes - o) < 32768u ? (bytes - o) : 32768u, bar);
-    }
-    mbar_wait(bar, 0);
-    c.tsm = smem_addr(tsm); c.tsm_kind = KIND;
+    stage_tables<G>(a, tile + mix_tile_floats(OUT, NT), bar, c);
   }
-  c.wt = a.wt; c.dl = a.dline; c.V = a.V; c.v = v; c.sr = a.sr; c.sd64 = a.sd64; c.sd32 = a.sd32;
-  c.rp = a.params; c.rs0 = a.state0; c.ru = a.uniform; c.dl_total = a.dl_floats;
   if (active) {
     Loader l{a.params, a.state, a.uniform, a.V, v, 0u, 0u, 0u, 0u};
     G::load(r, l);
@@ -89,73 +75,23 @@ __global__ void __launch_bounds__(NT, FDSP_MIN_CTAS) bank_kernel_rt(const BankAr
     for (int e = (int)tid; e < IN * 64; e += NT) s_in[e] = (e & 63) < nb ? __ldcv(&rt.ctl->in[e >> 6][e & 63]) : 0.0f;
     __syncthreads();
     // ---- one block, as bank_kernel evaluates it (MODE 2)
-    const int nfull = nb & ~7;
-    c.n = nb;
 #pragma unroll 1
     for (int s0 = 0; s0 < nb; s0 += TS) {
       const int s1 = (s0 + TS) < nb ? (s0 + TS) : nb;
       if (active) {
-        const int gend = s1 < nfull ? s1 : nfull;
-        c.rem = false;
-#pragma unroll 1
-        for (int g = s0; g < gend; g += 8) {
-          if constexpr (GROUP) {
-            Fr8<IN> in8; Fr8<OUT> o8;
-#pragma unroll
-            for (int k = 0; k < IN; k++) {
-#pragma unroll
-              for (int j = 0; j < 8; j++) in8.v[k][j] = s_in[k * 64 + g + j];
-            }
-            c.i = g; c.first = true;
-            group_step<G>(r, c, in8, o8);
-#pragma unroll
-            for (int k = 0; k < OUT; k++) {
-#pragma unroll
-              for (int j = 0; j < 8; j++) tile[(k * TS + (g - s0) + j) * (NT + 1) + tid] = o8.v[k][j];
-            }
-          } else {
-#pragma unroll(UNROLL)
-            for (int j = 0; j < 8; j++) {
-              Fr<IN> in; Fr<OUT> o;
-#pragma unroll
-              for (int k = 0; k < IN; k++) in.v[k] = s_in[k * 64 + g + j];
-              c.i = g + j; c.first = (j == 0);
-              G::template step<false>(r, c, in, o);
-#pragma unroll
-              for (int k = 0; k < OUT; k++) tile[(k * TS + (g - s0) + j) * (NT + 1) + tid] = o.v[k];
-            }
-          }
-        }
-        if (s1 == nb) {  // end of the block: wrap up the SIMD part, then the (size & 7) tail through the tick path
-          G::end_simd(r);
-          c.rem = true; c.first = false;
-#pragma unroll 1
-          for (int i = nfull; i < nb; i++) {
-            Fr<IN> in; Fr<OUT> o;
-#pragma unroll
-            for (int k = 0; k < IN; k++) in.v[k] = s_in[k * 64 + i];
-            c.i = i;
-            G::template step<false>(r, c, in, o);
-#pragma unroll
-            for (int k = 0; k < OUT; k++) tile[(k * TS + (i - s0)) * (NT + 1) + tid] = o.v[k];
-          }
-        }
+        auto put = [&](int k, int i, float y) { tile[(k * TS + (i - s0)) * (NT + 1) + tid] = y; };
+        walk_block<G>(r, c, nb, s0, s1, [&](int k, int i, int j) { return s_in[k * 64 + i + j]; }, put, [](int, int, const float (&)[8]) {}, put);
       }
-      // CTA partial mix: the association of bank_kernel (two threads per row, four interleaved accumulators each, low half + high half)
+      // CTA partial mix: the association of bank_kernel (mix_order.h)
       __syncthreads();
-      constexpr int HALF = NT / 2, QN = HALF / 4, ROWS = OUT * TS;
+      constexpr int HALF = NT / 2, ROWS = OUT * TS;
       const int h = (int)(tid & 1u);
-      const int c0 = h * HALF + (h * QN) % HALF, c1 = h * HALF + (QN + h * QN) % HALF, c2 = h * HALF + (2 * QN + h * QN) % HALF, c3 = h * HALF + (3 * QN + h * QN) % HALF;
 #pragma unroll 1
       for (int eb = (int)(tid >> 5) * 16; eb < ROWS; eb += HALF) {
         const int e = eb + (int)((tid & 31u) >> 1);
         const bool ok = e < ROWS;
         const int k = e / TS, i = e - k * TS;
-        const float* row = tile + (ok ? e : 0) * (NT + 1);
-        float a0 = row[c0], a1 = row[c1], a2 = row[c2], a3 = row[c3];
-#pragma unroll
-        for (int q = 1; q < QN; q++) { a0 += row[c0 + q]; a1 += row[c1 + q]; a2 += row[c2 + q]; a3 += row[c3 + q]; }
-        const float s = (a0 + a1) + (a2 + a3);
+        const float s = cta_half_row_sum<NT>(tile + (ok ? e : 0) * (NT + 1), h);
         const float other = __shfl_xor_sync(0xffffffffu, s, 1);
         if (ok && h == 0 && s0 + i < s1) a.partial[((size_t)blockIdx.x * OUT + k) * 64 + s0 + i] = s + other;
       }
@@ -168,23 +104,11 @@ __global__ void __launch_bounds__(NT, FDSP_MIN_CTAS) bank_kernel_rt(const BankAr
     __syncthreads();
     if (s_last) {
       __threadfence();
-      // CTA-order left fold of the partials (= mix_reduce_kernel, bit for bit). The loads of 8 CTAs are issued together, the adds stay in
-      // order. (A version that staged the partials in shared memory first measured SLOWER — 44.5 vs 23.4 us per block at 148 CTAs: one CTA
-      // cannot keep enough loads in flight to win back the extra pass.)
+      // CTA-order left fold of the partials (= mix_reduce_kernel, bit for bit). (A version that staged the partials in shared memory first
+      // measured SLOWER — 44.5 vs 23.4 us per block at 148 CTAs: one CTA cannot keep enough loads in flight to win back the extra pass.)
       for (uint32_t e = tid; e < (uint32_t)OUT * (uint32_t)nb; e += NT) {
         const uint32_t ch = e / (uint32_t)nb, t = e - ch * (uint32_t)nb;
-        const float* p0 = a.partial + (size_t)ch * 64 + t;
-        float s = __ldcg(p0);
-        uint32_t b = 1;
-        for (; b + 8 <= gridDim.x; b += 8) {
-          float x[8];
-#pragma unroll
-          for (int u = 0; u < 8; u++) x[u] = __ldcg(p0 + (size_t)(b + u) * OUT * 64);
-#pragma unroll
-          for (int u = 0; u < 8; u++) s += x[u];
-        }
-        for (; b < gridDim.x; b++) s += __ldcg(p0 + (size_t)b * OUT * 64);
-        rt.ctl->out[ch][t] = s;
+        rt.ctl->out[ch][t] = cta_order_fold(a.partial + (size_t)ch * 64 + t, (size_t)OUT * 64, gridDim.x, [](const float* p) { return __ldcg(p); });
       }
       __threadfence_system();
       __syncthreads();

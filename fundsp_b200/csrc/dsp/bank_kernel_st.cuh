@@ -39,7 +39,7 @@ template <class G, int NT, int MODE, bool TB, int I> struct StRun {
   static constexpr int IN = S::IN, OUT = S::OUT;
   static constexpr int TS = (MODE & 2) ? mix_tile_samples(G::OUT) : 64;
   static constexpr int HS = st_hand_samples(G::OUT, (MODE & 2) != 0);
-  static constexpr bool GROUP = GroupPlan<S>::ok && GroupPlan<S>::code <= FDSP_GROUP_COST && !FDSP_NO_GROUP;
+  static constexpr bool GROUP = VoiceForm<S>::group;
   // ring of boundary b (between stage b and b + 1), warp w: [slot][MID_b][HS][32]
   static FDSP_DEV float* ring_of(float* hand, int before_mid, uint32_t w, uint32_t lane, int mid) {
     return hand + ((size_t)before_mid * NT + (size_t)w * mid * 32) * ST_NSLOT * HS + lane;
@@ -53,10 +53,8 @@ template <class G, int NT, int MODE, bool TB, int I> struct StRun {
   static FDSP_DEV void run(const BankArgs& a, float* tile, float* hand, uint32_t bar0, CtxT<TB>& c0, uint32_t lt, uint32_t v, bool active) {
     // a stage built around a heavy leaf is one serial chain per lane: its 8 steps of a group are unrolled outright (static register indices, the
     // group's inputs loaded up front) instead of the rotating loop the one-warp-does-everything kernel uses to keep its instruction stream small
-    CtxT<TB, SpineHeavy<S>::value> c;
-    c.wt = c0.wt; c.tsm = c0.tsm; c.tsm_kind = c0.tsm_kind; c.dl = c0.dl; c.V = c0.V; c.v = c0.v; c.sr = c0.sr; c.sd64 = c0.sd64; c.sd32 = c0.sd32;
-    c.rp = c0.rp; c.rs0 = c0.rs0; c.ru = c0.ru; c.dl_total = c0.dl_total;
-    c.i = 0; c.n = 0; c.first = false; c.rem = false;
+    CtxT<TB, SpineHeavy<S>::value> c = voice_ctx<TB, SpineHeavy<S>::value>(a, v);
+    c.tsm = c0.tsm; c.tsm_kind = c0.tsm_kind;
     const uint32_t w = lt >> 5, lane = lt & 31u;
     constexpr int MIDI = FIRST ? 1 : IN, MIDO = LAST ? 1 : OUT;
     // barriers: index 1 + ((b * NW + w) * NSLOT + slot) * 2 (+1 = empty)
@@ -182,22 +180,16 @@ template <class G, int NT, int MODE, bool TB, int I> struct StRun {
           if (!LAST) mbar_arrive(full_bar(I, slot));
         }
         if (LAST && (MODE & 2)) {
-          // CTA partial mix by the last stage alone (named barrier 1): same association as bank_kernel — two threads per row,
-          // four interleaved accumulators each, low half + high half
+          // CTA partial mix by the last stage alone (named barrier 1): same association as bank_kernel (mix_order.h)
           bar_named(1, NT);
-          constexpr int HALF = NT / 2, QN = HALF / 4 > 0 ? HALF / 4 : 1, ROWS = G::OUT * TS;
+          constexpr int HALF = NT / 2, ROWS = G::OUT * TS;
           const int h = (int)(lt & 1u);
-          const int c0 = h * HALF + (h * QN) % HALF, c1 = h * HALF + (QN + h * QN) % HALF, c2 = h * HALF + (2 * QN + h * QN) % HALF, c3 = h * HALF + (3 * QN + h * QN) % HALF;
 #pragma unroll 1
           for (int eb = (int)(lt >> 5) * 16; eb < ROWS; eb += HALF) {
             const int e = eb + (int)((lt & 31u) >> 1);
             const bool ok = e < ROWS;
             const int k = e / TS, i = e - k * TS;
-            const float* row = tile + (ok ? e : 0) * (NT + 1);
-            float a0 = row[c0], a1 = row[c1], a2 = row[c2], a3 = row[c3];
-#pragma unroll
-            for (int q = 1; q < QN; q++) { a0 += row[c0 + q]; a1 += row[c1 + q]; a2 += row[c2 + q]; a3 += row[c3 + q]; }
-            const float s = (a0 + a1) + (a2 + a3);
+            const float s = cta_half_row_sum<NT>(tile + (ok ? e : 0) * (NT + 1), h);
             const float other = __shfl_xor_sync(0xffffffffu, s, 1);
             if (ok && h == 0 && m0 + i < m1) a.partial[((size_t)blockIdx.x * G::OUT + k) * a.n + t0 + m0 + i] = s + other;
           }
@@ -239,22 +231,8 @@ __global__ void __launch_bounds__(StagePlan<G>::K * NT, 1) bank_kernel_st(const 
     for (int q = 1; q < NBAR; q++) mbar_init(bar0 + 8u * q, 32);
   }
   __syncthreads();
-  CtxT<TB> c;
-  c.tsm = 0u; c.tsm_kind = -1;
-  if (TB) {
-    constexpr int KIND = WaveKind<G>::value >= 0 ? WaveKind<G>::value : 0;
-    float* tsm = hand + st_hand_floats<G>(NT, (MODE & 2) != 0);
-    const uint32_t bytes = (uint32_t)a.wt[KIND].total * 4u;
-    if (tid == 0) {
-      mbar_expect_tx(bar0, bytes);
-      const char* src = reinterpret_cast<const char*>(a.wt[KIND].data);
-      for (uint32_t o = 0; o < bytes; o += 32768u) bulk_g2s(smem_addr(tsm) + o, src + o, (bytes - o) < 32768u ? (bytes - o) : 32768u, bar0);
-    }
-    mbar_wait(bar0, 0);
-    c.tsm = smem_addr(tsm); c.tsm_kind = KIND;
-  }
-  c.wt = a.wt; c.dl = a.dline; c.V = a.V; c.v = v; c.sr = a.sr; c.sd64 = a.sd64; c.sd32 = a.sd32;
-  c.rp = a.params; c.rs0 = a.state0; c.ru = a.uniform; c.dl_total = a.dl_floats;
+  CtxT<TB> c = voice_ctx<TB>(a, v);
+  if (TB) stage_tables<G>(a, hand + st_hand_floats<G>(NT, (MODE & 2) != 0), bar0, c);
   st_dispatch<G, NT, MODE, TB, 0>(stage, a, tile, hand, bar0, c, lt, v, active);
 }
 

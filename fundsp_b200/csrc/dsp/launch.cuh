@@ -19,9 +19,8 @@ template <class G, int MODE, bool TB> cudaError_t launch_one(const BankArgs& a, 
   bank_kernel<G, NT, MODE, TB><<<grid, NT, smem, st>>>(a);
   return cudaGetLastError();
 }
-template <class G, bool TB> cudaError_t launch_mode(const BankArgs& a, int mode, size_t table_bytes, cudaStream_t st) {
+template <class G, bool TB> cudaError_t launch_mode(const BankArgs& a, int mode, size_t smem, cudaStream_t st) {
   const unsigned vpc = a.vpc ? a.vpc : (unsigned)NT, grid = (a.V + vpc - 1) / vpc;
-  const size_t smem = ((mode & 2) ? sizeof(float) * mix_tile_floats(G::OUT, NT) : 0) + (TB ? table_bytes : 0);
   switch (mode & 3) {
     case 1: return launch_one<G, 1, TB>(a, grid, smem, st);
     case 2: return launch_one<G, 2, TB>(a, grid, smem, st);
@@ -42,11 +41,8 @@ template <class G, int NTV, int MODE, bool TB> cudaError_t launch_st_one(const B
     return cudaErrorInvalidValue;
   }
 }
-template <class G, int NTV, bool TB> cudaError_t launch_st_mode(const BankArgs& a, int mode, size_t table_bytes, cudaStream_t st) {
+template <class G, int NTV, bool TB> cudaError_t launch_st_mode(const BankArgs& a, int mode, size_t smem, cudaStream_t st) {
   const unsigned vpc = a.vpc ? a.vpc : (unsigned)NTV, grid = (a.V + vpc - 1) / vpc;
-  const bool mix = (mode & 2) != 0;
-  const size_t smem = (mix ? sizeof(float) * mix_tile_floats(G::OUT, NTV) : 0) + sizeof(float) * st_hand_floats<G>(NTV, mix) + (TB ? table_bytes : 0);
-  if (smem > 227 * 1024) return cudaErrorInvalidValue;
   switch (mode & 3) {
     case 1: return launch_st_one<G, NTV, 1, TB>(a, grid, smem, st);
     case 2: return launch_st_one<G, NTV, 2, TB>(a, grid, smem, st);
@@ -54,25 +50,20 @@ template <class G, int NTV, bool TB> cudaError_t launch_st_mode(const BankArgs& 
     default: return cudaErrorInvalidValue;
   }
 }
+// table_bytes > 0 asks for the shared-memory wavetable variant (only taken when G reads a wavetable and it fits, launch_smem)
+template <class G> size_t table_bytes_of(size_t table_bytes) { return WaveKind<G>::value >= 0 ? table_bytes : 0; }
 // stage width: 32 voices per CTA when the launch asks for at most 32 (a.vpc), else 128
 template <class G> cudaError_t launch_st_t(const BankArgs& a, int mode, size_t table_bytes, cudaStream_t st) {
   constexpr bool WT = WaveKind<G>::value >= 0;
   const bool narrow = a.vpc && a.vpc <= 32u;
-  const bool mix = (mode & 2) != 0;
-  const int ntv = narrow ? 32 : 128;
-  // tables in shared memory only when they fit beside the mix tile and the hand-off rings (else they are read through L1 / L2)
-  const size_t base = (mix ? sizeof(float) * mix_tile_floats(G::OUT, ntv) : 0) + sizeof(float) * st_hand_floats<G>(ntv, mix);
-  const bool tb = WT && table_bytes > 0 && base + table_bytes <= 227 * 1024;
-  if (narrow) return tb ? launch_st_mode<G, 32, WT>(a, mode, table_bytes, st) : launch_st_mode<G, 32, false>(a, mode, 0, st);
-  return tb ? launch_st_mode<G, 128, WT>(a, mode, table_bytes, st) : launch_st_mode<G, 128, false>(a, mode, 0, st);
+  const LaunchSmem L = launch_smem(G::OUT, narrow ? 32 : 128, MidSum<typename StagePlan<G>::stages>::value, mode, table_bytes_of<G>(table_bytes));
+  if (L.smem > SMEM_BLOCK_MAX) return cudaErrorInvalidValue;
+  if (narrow) return L.tb ? launch_st_mode<G, 32, WT>(a, mode, L.smem, st) : launch_st_mode<G, 32, false>(a, mode, L.smem, st);
+  return L.tb ? launch_st_mode<G, 128, WT>(a, mode, L.smem, st) : launch_st_mode<G, 128, false>(a, mode, L.smem, st);
 }
-// table_bytes > 0 asks for the shared-memory wavetable variant (only meaningful when G reads a wavetable and it fits).
 template <class G> cudaError_t launch_t(const BankArgs& a, int mode, size_t table_bytes, cudaStream_t st) {
-  if (WaveKind<G>::value >= 0 && table_bytes > 0) {
-    const size_t smem = ((mode & 2) ? sizeof(float) * mix_tile_floats(G::OUT, NT) : 0) + table_bytes;
-    if (smem <= 227 * 1024) return launch_mode<G, (WaveKind<G>::value >= 0)>(a, mode, table_bytes, st);
-  }
-  return launch_mode<G, false>(a, mode, 0, st);
+  const LaunchSmem L = launch_smem(G::OUT, NT, 0, mode, table_bytes_of<G>(table_bytes));
+  return L.tb ? launch_mode<G, (WaveKind<G>::value >= 0)>(a, mode, L.smem, st) : launch_mode<G, false>(a, mode, L.smem, st);
 }
 // resident process() kernel (bank_kernel_rt.cuh): one launch serves 64-sample blocks on a doorbell until it is told to leave
 template <class G, bool TB> cudaError_t launch_rt_one(const BankArgs& a, const RtArgs& rt, size_t smem, cudaStream_t st) {
@@ -85,9 +76,8 @@ template <class G, bool TB> cudaError_t launch_rt_one(const BankArgs& a, const R
   return cudaGetLastError();
 }
 template <class G> cudaError_t launch_rt_t(const BankArgs& a, const RtArgs& rt, size_t table_bytes, cudaStream_t st) {
-  const size_t tile = sizeof(float) * mix_tile_floats(G::OUT, NT);
-  if (WaveKind<G>::value >= 0 && table_bytes > 0 && tile + table_bytes <= 227 * 1024) return launch_rt_one<G, (WaveKind<G>::value >= 0)>(a, rt, tile + table_bytes, st);
-  return launch_rt_one<G, false>(a, rt, tile, st);
+  const LaunchSmem L = launch_smem(G::OUT, NT, 0, 2, table_bytes_of<G>(table_bytes));
+  return L.tb ? launch_rt_one<G, (WaveKind<G>::value >= 0)>(a, rt, L.smem, st) : launch_rt_one<G, false>(a, rt, L.smem, st);
 }
 template <class G> int wave_kind_t() { return WaveKind<G>::value; }
 inline int threads_t() { return NT; }

@@ -99,15 +99,11 @@ template <class G> struct StagePlan {
   static_assert(ChainSum<stages>::np == G::NP && ChainSum<stages>::ns == G::NS && ChainSum<stages>::nu == G::NU, "staging must keep the word layout");
   static_assert(ChainAt<0, stages>::type::IN == G::IN && ChainAt<K - 1, stages>::type::OUT == G::OUT, "staging must keep the program's arity");
 };
-// floats of hand-off ring per voice slot of the CTA (all K-1 boundaries, NSLOT slots of HS samples)
-constexpr int ST_NSLOT = 2;
-FDSP_HDC constexpr int st_hand_samples(int outs, bool mix) { return mix && mix_tile_samples(outs) < 16 ? mix_tile_samples(outs) : 16; }
 template <class C> struct MidSum { static constexpr int value = 0; };
 template <class A, class B, class... T> struct MidSum<Chain<A, B, T...>> { static constexpr int value = A::OUT + MidSum<Chain<B, T...>>::value; };
 template <int I, class C> struct MidBefore { static constexpr int value = 0; };   // sum of OUT of stages < I
 template <int I, class H, class... T> struct MidBefore<I, Chain<H, T...>> { static constexpr int value = I == 0 ? 0 : H::OUT + MidBefore<(I > 0 ? I - 1 : 0), Chain<T...>>::value; };
-template <class G> FDSP_HDC constexpr size_t st_hand_floats(int nt, bool mix) {
-  return (size_t)ST_NSLOT * MidSum<typename StagePlan<G>::stages>::value * st_hand_samples(G::OUT, mix) * nt;
-}
+// floats of hand-off ring of the CTA (all K-1 boundaries)
+template <class G> FDSP_HDC constexpr size_t st_hand_floats(int nt, bool mix) { return st_ring_floats(G::OUT, MidSum<typename StagePlan<G>::stages>::value, nt, mix); }
 
 }  // namespace fdsp

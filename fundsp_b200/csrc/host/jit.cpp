@@ -197,11 +197,10 @@ struct JitProgram : Program {
   }
   cudaError_t launch_rt(const BankArgs& a, const RtArgs& rt, size_t table_bytes, cudaStream_t st) const override {
     const Api& A = api();
-    const size_t tile = sizeof(float) * mix_tile_floats(OUT, threads);
-    const int tb = (wave_kind >= 0 && table_bytes > 0 && tile + table_bytes <= 227 * 1024) ? 1 : 0;
-    CUfunction f = variant(2, tb, -1);
+    const LaunchSmem L = launch_smem(OUT, threads, 0, 2, wave_kind >= 0 ? table_bytes : 0);
+    const size_t smem = L.smem;
+    CUfunction f = variant(2, L.tb, -1);
     if (!f) return cudaErrorInvalidDeviceFunction;
-    const size_t smem = tile + (tb ? table_bytes : 0);
     if (smem > 48 * 1024 && A.FuncSetAttribute(f, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, (int)smem) != CUDA_SUCCESS) return cudaErrorInvalidValue;
     if (launch_carveout() >= 0) A.FuncSetAttribute(f, CU_FUNC_ATTRIBUTE_PREFERRED_SHARED_MEMORY_CARVEOUT, launch_carveout());
     BankArgs args = a; RtArgs r = rt;
@@ -215,13 +214,10 @@ struct JitProgram : Program {
     mode &= 3;
     if (mode == 0 || stages < 2) return cudaErrorInvalidValue;
     const int width = (a.vpc && a.vpc <= 32u) ? 32 : 128;
-    const bool mix = (mode & 2) != 0;
-    const int hs = mix && mix_tile_samples(OUT) < 16 ? mix_tile_samples(OUT) : 16;   // st_hand_samples
-    const size_t base = (mix ? sizeof(float) * mix_tile_floats(OUT, width) : 0) + sizeof(float) * 2 /*ST_NSLOT*/ * (size_t)mid_sum * hs * width;
-    const int tb = (wave_kind >= 0 && table_bytes > 0 && base + table_bytes <= 227 * 1024) ? 1 : 0;
-    const size_t smem = base + (tb ? table_bytes : 0);
-    if (smem > 227 * 1024) return cudaErrorInvalidValue;
-    CUfunction f = variant(mode, tb, width);
+    const LaunchSmem L = launch_smem(OUT, width, mid_sum, mode, wave_kind >= 0 ? table_bytes : 0);
+    const size_t smem = L.smem;
+    if (smem > SMEM_BLOCK_MAX) return cudaErrorInvalidValue;
+    CUfunction f = variant(mode, L.tb, width);
     if (!f) return cudaErrorInvalidDeviceFunction;
     if (smem > 48 * 1024 && A.FuncSetAttribute(f, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, (int)smem) != CUDA_SUCCESS) return cudaErrorInvalidValue;
     if (launch_carveout() >= 0) A.FuncSetAttribute(f, CU_FUNC_ATTRIBUTE_PREFERRED_SHARED_MEMORY_CARVEOUT, launch_carveout());
@@ -235,11 +231,10 @@ struct JitProgram : Program {
     const Api& A = api();
     mode &= 3;
     if (mode == 0) return cudaErrorInvalidValue;
-    const size_t tile = (mode & 2) ? sizeof(float) * mix_tile_floats(OUT, threads) : 0;
-    int tb = (wave_kind >= 0 && table_bytes > 0 && tile + table_bytes <= 227 * 1024) ? 1 : 0;
-    CUfunction f = variant(mode, tb);
+    const LaunchSmem L = launch_smem(OUT, threads, 0, mode, wave_kind >= 0 ? table_bytes : 0);
+    const size_t smem = L.smem;
+    CUfunction f = variant(mode, L.tb);
     if (!f) return cudaErrorInvalidDeviceFunction;
-    const size_t smem = tile + (tb ? table_bytes : 0);
     if (smem > 48 * 1024 && A.FuncSetAttribute(f, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, (int)smem) != CUDA_SUCCESS) return cudaErrorInvalidValue;
     if (launch_carveout() >= 0) A.FuncSetAttribute(f, CU_FUNC_ATTRIBUTE_PREFERRED_SHARED_MEMORY_CARVEOUT, launch_carveout());
     BankArgs args = a;

@@ -1,8 +1,8 @@
 // TEST INFRASTRUCTURE — host emulation of ONE voice of a fused device program.
 //
 // Compiles the DEVICE node library (fundsp_b200/csrc/dsp/nodes.cuh) for the CPU (FDSP_HOST_EMUL shims in math.cuh) and walks it
-// through the same block structure as bank_kernel (8-sample groups, end_simd, tick-path tail), so that the CPU-only test suite
-// can compare the device templates against the oracle bit for bit. It is never linked into the product and is not a fallback:
+// through a block with the kernels' own walk_block (dsp/voice_block.cuh: 8-sample groups, end_simd, tick-path tail), so that the
+// CPU-only test suite can compare the device templates against the oracle bit for bit. It is never linked into the product and is not a fallback:
 // the product library has no CPU DSP path. Build: g++ -std=c++17 -O1 -ffp-contract=off -DGRAPH='<type expression>' device_emul.cpp
 //
 // stdin-free protocol: argv[1] = input blob, argv[2] = output file.
@@ -14,7 +14,7 @@
 #include <cstdlib>
 #include <vector>
 
-#include "../../fundsp_b200/csrc/dsp/nodes.cuh"
+#include "../../fundsp_b200/csrc/dsp/voice_block.cuh"
 #ifdef STAGED
 #include "../../fundsp_b200/csrc/dsp/stage_plan.cuh"
 #endif
@@ -30,41 +30,11 @@ template <int I> struct StageEmul {
   static constexpr int K = StagePlan<G>::K;
   typedef typename ChainAt<(I < K ? I : 0), STG>::type S;
   template <int J> static void skip(Loader& l) { if constexpr (J < I) { typename ChainAt<J, STG>::type::R sk; ChainAt<J, STG>::type::load(sk, l); skip<J + 1>(l); } }
-  static void block(typename S::R& r, CtxT<false> c0, int nb, const float* in /*[IN][64]*/, float* out /*[OUT][64]*/) {
-    constexpr int IN = S::IN, OUT = S::OUT;
+  static void block(typename S::R& r, const BankArgs& a, int nb, const float* in /*[IN][64]*/, float* out /*[OUT][64]*/) {
     // like bank_kernel_st: a stage built around a heavy leaf runs the leaf's 8 steps fully unrolled (and takes its steady-group path)
-    CtxT<false, SpineHeavy<S>::value> c;
-    c.wt = c0.wt; c.tsm = c0.tsm; c.tsm_kind = c0.tsm_kind; c.dl = c0.dl; c.V = c0.V; c.v = c0.v; c.sr = c0.sr; c.sd64 = c0.sd64; c.sd32 = c0.sd32;
-    c.rp = c0.rp; c.rs0 = c0.rs0; c.ru = c0.ru; c.dl_total = c0.dl_total; c.i = 0; c.n = 0; c.first = false; c.rem = false;
-    constexpr bool GROUP = GroupPlan<S>::ok && GroupPlan<S>::code <= 256;
-    const int nfull = nb & ~7;
-    c.n = nb; c.rem = false;
-    for (int g = 0; g < nfull; g += 8) {
-      if (GROUP) {
-        Fr8<IN> in8; Fr8<OUT> o8;
-        for (int k = 0; k < IN; k++) for (int j = 0; j < 8; j++) in8.v[k][j] = in[k * 64 + g + j];
-        c.i = g; c.first = true;
-        group_step<S>(r, c, in8, o8);
-        for (int k = 0; k < OUT; k++) for (int j = 0; j < 8; j++) out[k * 64 + g + j] = o8.v[k][j];
-      } else {
-        for (int j = 0; j < 8; j++) {
-          Fr<IN> a; Fr<OUT> b;
-          for (int k = 0; k < IN; k++) a.v[k] = in[k * 64 + g + j];
-          c.i = g + j; c.first = (j == 0);
-          S::template step<false>(r, c, a, b);
-          for (int k = 0; k < OUT; k++) out[k * 64 + g + j] = b.v[k];
-        }
-      }
-    }
-    S::end_simd(r);
-    c.rem = true; c.first = false;
-    for (int i = nfull; i < nb; i++) {
-      Fr<IN> a; Fr<OUT> b;
-      for (int k = 0; k < IN; k++) a.v[k] = in[k * 64 + i];
-      c.i = i;
-      S::template step<false>(r, c, a, b);
-      for (int k = 0; k < OUT; k++) out[k * 64 + i] = b.v[k];
-    }
+    CtxT<false, SpineHeavy<S>::value> c = voice_ctx<false, SpineHeavy<S>::value>(a, 0);
+    auto put = [&](int k, int i, float y) { out[k * 64 + i] = y; };
+    walk_block<S>(r, c, nb, 0, nb, [&](int k, int i, int j) { return in[k * 64 + i + j]; }, put, [](int, int, const float (&)[8]) {}, put);
   }
 };
 template <int I> struct StageRegs { typename StageEmul<I>::S::R r; StageRegs<I + 1> next; };
@@ -78,10 +48,10 @@ template <int I> static void staged_load(StageRegs<I>& regs, const uint32_t* P, 
     staged_load<I + 1>(regs.next, P, S, U, dl);
   }
 }
-template <int I> static void staged_block(StageRegs<I>& regs, const CtxT<false>& c, int nb, float* a, float* b) {
+template <int I> static void staged_block(StageRegs<I>& regs, const BankArgs& args, int nb, float* a, float* b) {
   if constexpr (I < StagePlan<G>::K) {
-    StageEmul<I>::block(regs.r, c, nb, a, b);
-    staged_block<I + 1>(regs.next, c, nb, b, a);   // ping-pong: the output of stage I is the input of stage I + 1
+    StageEmul<I>::block(regs.r, args, nb, a, b);
+    staged_block<I + 1>(regs.next, args, nb, b, a);   // ping-pong: the output of stage I is the input of stage I + 1
   }
 }
 #endif
@@ -115,26 +85,25 @@ int main(int argc, char** argv) {
     }
   }
   fclose(f);
+  BankArgs args = {};   // one voice: the launch arguments the block context is built from
+  args.params = P.data(); args.state = S.data(); args.uniform = U.data(); args.state0 = S.data(); args.wt = wt; args.V = 1;
+  args.sr = (float)sr; args.sd64 = (float)(1.0 / sr); args.sd32 = 1.0f / (float)sr;
 
 #ifdef STAGED
   {
     static_assert(StagePlan<G>::K >= 2, "the graph has no stage plan (no heavy leaf on its spine)");
     fprintf(stderr, "stages=%d\n", StagePlan<G>::K);
-    CtxT<false> c;
-    c.wt = wt; c.tsm = 0u; c.tsm_kind = -1; c.V = 1; c.v = 0;
-    c.sr = (float)sr; c.sd64 = (float)(1.0 / sr); c.sd32 = 1.0f / (float)sr;
-    c.rp = P.data(); c.rs0 = S.data(); c.ru = U.data(); c.dl_total = 0u;
     StageRegs<0> regs; uint32_t dl = 0;
     staged_load<0>(regs, P.data(), S.data(), U.data(), dl);
     std::vector<float> dline((size_t)dl + 1, 0.0f);
     fprintf(stderr, "dl=%u\n", dl);
-    c.dl = dline.data();
+    args.dline = dline.data(); args.dl_floats = dl;
     constexpr int CH = 64;   // widest boundary the ping-pong buffers hold
     std::vector<float> bufa(CH * 64), bufb(CH * 64);
     for (uint32_t t0 = 0; t0 < n; t0 += 64) {
       const int nb = (n - t0) < 64u ? (int)(n - t0) : 64;
       for (uint32_t k = 0; k < nin; k++) for (int i = 0; i < nb; i++) bufa[k * 64 + i] = in[(size_t)k * n + t0 + i];
-      staged_block<0>(regs, c, nb, bufa.data(), bufb.data());
+      staged_block<0>(regs, args, nb, bufa.data(), bufb.data());
       const float* res = (StagePlan<G>::K & 1) ? bufb.data() : bufa.data();
       for (int k = 0; k < G::OUT; k++) for (int i = 0; i < nb; i++) out[(size_t)k * n + t0 + i] = res[k * 64 + i];
     }
@@ -146,53 +115,21 @@ int main(int argc, char** argv) {
   }
 #endif
   typename G::R r;
-  CtxT<false> c;
-  c.wt = wt; c.tsm = 0u; c.tsm_kind = -1; c.V = 1; c.v = 0;
-  c.sr = (float)sr; c.sd64 = (float)(1.0 / sr); c.sd32 = 1.0f / (float)sr;
-  const std::vector<uint32_t> S0 = S;   // the reset image (Event<X> of a looping sequencer resets its unit from it)
-  c.rp = P.data(); c.rs0 = S0.data(); c.ru = U.data(); c.dl_total = 0u;
   Loader l{P.data(), S.data(), U.data(), 1u, 0u, 0u, 0u, 0u, 0u};
   G::load(r, l);
   if (l.pi > np || l.si > ns || l.ui > nu) { fprintf(stderr, "word layout mismatch: consumed %u/%u/%u of %u/%u/%u\n", l.pi, l.si, l.ui, np, ns, nu); return 8; }
   std::vector<float> dline((size_t)l.dl + 1, 0.0f);
   fprintf(stderr, "dl=%u\n", l.dl);   // the delay-line floats the device program claims (the host must allocate exactly this)
-  c.dl = dline.data(); c.dl_total = l.dl;
-  constexpr int IN = G::IN, OUT = G::OUT;
-  constexpr bool GROUP = GroupPlan<G>::ok && GroupPlan<G>::code <= 256;   // bank_kernel's FDSP_GROUP_COST
+  args.dline = dline.data(); args.dl_floats = l.dl;
+  CtxT<false> c = voice_ctx<false>(args, 0);
   for (uint32_t t0 = 0; t0 < n; t0 += 64) {
     const int nb = (n - t0) < 64u ? (int)(n - t0) : 64;
-    const int nfull = nb & ~7;
-    c.n = nb; c.rem = false;
-    for (int g = 0; g < nfull; g += 8) {
-      if (GROUP) {
-        Fr8<IN> in8; Fr8<OUT> o8;
-        for (int k = 0; k < IN; k++) for (int j = 0; j < 8; j++) in8.v[k][j] = in[(size_t)k * n + t0 + g + j];
-        c.i = g; c.first = true;
-        group_step<G>(r, c, in8, o8);
-        for (int k = 0; k < OUT; k++) for (int j = 0; j < 8; j++) out[(size_t)k * n + t0 + g + j] = o8.v[k][j];
-      } else {
-        for (int j = 0; j < 8; j++) {
-          Fr<IN> a; Fr<OUT> b;
-          for (int k = 0; k < IN; k++) a.v[k] = in[(size_t)k * n + t0 + g + j];
-          c.i = g + j; c.first = (j == 0);
-          G::template step<false>(r, c, a, b);
-          for (int k = 0; k < OUT; k++) out[(size_t)k * n + t0 + g + j] = b.v[k];
-        }
-      }
-    }
-    G::end_simd(r);
-    c.rem = true; c.first = false;
-    for (int i = nfull; i < nb; i++) {
-      Fr<IN> a; Fr<OUT> b;
-      for (int k = 0; k < IN; k++) a.v[k] = in[(size_t)k * n + t0 + i];
-      c.i = i;
-      G::template step<false>(r, c, a, b);
-      for (int k = 0; k < OUT; k++) out[(size_t)k * n + t0 + i] = b.v[k];
-    }
+    auto put = [&](int k, int i, float y) { out[(size_t)k * n + t0 + i] = y; };
+    walk_block<G>(r, c, nb, 0, nb, [&](int k, int i, int j) { return in[(size_t)k * n + t0 + i + j]; }, put, [](int, int, const float (&)[8]) {}, put);
   }
   FILE* o = fopen(argv[2], "wb");
   if (!o) return 9;
-  fwrite(out.data(), 4, (size_t)OUT * n, o);
+  fwrite(out.data(), 4, (size_t)G::OUT * n, o);
   fclose(o);
   return 0;
 }

@@ -1,10 +1,14 @@
 // TEST INFRASTRUCTURE — one graph class of the mock "GPU" (tests/cpp/mock/registry_mock.cpp): the DEVICE node library compiled for the
-// CPU (FDSP_HOST_EMUL) and walked through bank_kernel's per-thread block structure for every voice of a launch, reading and writing
-// the same argument block (BankArgs) the real kernel gets. The CTA mix tile is replaced by a voice-order sum per CTA (the association
-// differs from the GPU's, as the GPU's differs from a left fold: mixes are compared with the tolerance of DESIGN.md §4).
+// CPU (FDSP_HOST_EMUL) and walked through the kernels' own walk_block (dsp/voice_block.cuh) for every voice of a launch, reading and
+// writing the same argument block (BankArgs) the real kernel gets. The per-CTA mix partials fold each row of a CTA's voice outputs in
+// the kernels' association (dsp/mix_order.h), so they equal the GPU's bit for bit.
 // Build: g++ -std=c++17 -O1 -ffp-contract=off -shared -fPIC -DGRAPH='<type expression>' -I fundsp_b200/csrc emul_module.cpp
 #define FDSP_HOST_EMUL 1
-#include "dsp/nodes.cuh"
+#include <algorithm>
+#include <vector>
+
+#include "dsp/mix_order.h"
+#include "dsp/voice_block.cuh"
 
 using namespace fdsp;
 typedef GRAPH G;
@@ -19,64 +23,39 @@ extern "C" int fdsp_emul_launch_ex(const BankArgs* ap, int mode, const float* pe
 extern "C" int fdsp_emul_launch(const BankArgs* ap, int mode) { return fdsp_emul_launch_ex(ap, mode, nullptr, 0); }
 extern "C" int fdsp_emul_launch_ex(const BankArgs* ap, int mode, const float* per_voice_in, uint64_t voice_stride) {
   const BankArgs& a = *ap;
-  constexpr int IN = G::IN, OUT = G::OUT;
-  constexpr bool GROUP = GroupPlan<G>::ok && GroupPlan<G>::code <= 256;   // bank_kernel's FDSP_GROUP_COST
-  const uint32_t vpc = a.vpc ? a.vpc : 128u, grid = (a.V + vpc - 1) / vpc;
+  constexpr int IN = G::IN, OUT = G::OUT, NT = 128;
+  const uint32_t vpc = a.vpc ? a.vpc : (uint32_t)NT, grid = (a.V + vpc - 1) / vpc;
   if ((mode & 2) && !a.partial) return 1;
   if ((mode & 1) && !a.out) return 2;
-  if (mode & 2) for (size_t e = 0; e < (size_t)grid * OUT * a.n; e++) a.partial[e] = 0.0f;
-  for (uint32_t v = 0; v < a.V; v++) {
-    typename G::R r;
-    CtxT<false> c;
-    c.wt = a.wt; c.tsm = 0u; c.tsm_kind = -1; c.dl = a.dline; c.V = a.V; c.v = v; c.sr = a.sr; c.sd64 = a.sd64; c.sd32 = a.sd32;
-    c.rp = a.params; c.rs0 = a.state0; c.ru = a.uniform; c.dl_total = a.dl_floats;
-    Loader l{a.params, a.state, a.uniform, a.V, v, 0u, 0u, 0u, 0u};
-    G::load(r, l);
-    const uint32_t b = v / vpc;
-    auto emit = [&](int k, uint32_t t, float y) {
-      if (mode & 1) a.out[(size_t)(a.row_map[v] + (uint32_t)k) * a.out_stride + a.out_offset + t] = y;
-      if (mode & 2) a.partial[((size_t)b * OUT + k) * a.n + t] += y;
-    };
-    for (uint32_t t0 = 0; t0 < a.n; t0 += 64) {
-      const int nb = (a.n - t0) < 64u ? (int)(a.n - t0) : 64;
-      const int nfull = nb & ~7;
-      const float* irow = (IN > 0) ? (per_voice_in ? per_voice_in + (size_t)v * voice_stride : a.in) + a.in_offset + t0 : nullptr;
-      c.n = nb; c.rem = false;
-      for (int g = 0; g < nfull; g += 8) {
-        if (GROUP) {
-          Fr8<IN> in8; Fr8<OUT> o8;
-          for (int k = 0; k < IN; k++) for (int j = 0; j < 8; j++) in8.v[k][j] = irow[(size_t)k * a.in_stride + g + j];
-          c.i = g; c.first = true;
-          group_step<G>(r, c, in8, o8);
-          for (int k = 0; k < OUT; k++) for (int j = 0; j < 8; j++) emit(k, t0 + g + j, o8.v[k][j]);
-        } else {
-          for (int j = 0; j < 8; j++) {
-            Fr<IN> x; Fr<OUT> y;
-            for (int k = 0; k < IN; k++) x.v[k] = irow[(size_t)k * a.in_stride + g + j];
-            c.i = g + j; c.first = (j == 0);
-            G::template step<false>(r, c, x, y);
-            for (int k = 0; k < OUT; k++) emit(k, t0 + g + j, y.v[k]);
-          }
-        }
+  if (vpc > (uint32_t)NT) return 3;
+  std::vector<float> tile((mode & 2) ? (size_t)OUT * a.n * NT : 0);   // one CTA's mix tile: row k * n + t, column = voice within the CTA
+  for (uint32_t b = 0; b < grid; b++) {
+    std::fill(tile.begin(), tile.end(), 0.0f);   // columns of absent voices stay zero
+    for (uint32_t v = b * vpc; v < a.V && v < (b + 1) * vpc; v++) {
+      typename G::R r;
+      CtxT<false> c = voice_ctx<false>(a, v);
+      Loader l{a.params, a.state, a.uniform, a.V, v, 0u, 0u, 0u, 0u};
+      G::load(r, l);
+      for (uint32_t t0 = 0; t0 < a.n; t0 += 64) {
+        const int nb = (a.n - t0) < 64u ? (int)(a.n - t0) : 64;
+        const float* irow = (IN > 0) ? (per_voice_in ? per_voice_in + (size_t)v * voice_stride : a.in) + a.in_offset + t0 : nullptr;
+        auto put = [&](int k, int i, float y) {
+          const uint32_t t = t0 + (uint32_t)i;
+          if (mode & 1) a.out[(size_t)(a.row_map[v] + (uint32_t)k) * a.out_stride + a.out_offset + t] = y;
+          if (mode & 2) tile[((size_t)k * a.n + t) * NT + (v - b * vpc)] = y;
+        };
+        walk_block<G>(r, c, nb, 0, nb, [&](int k, int i, int j) { return irow[(size_t)k * a.in_stride + i + j]; }, put, [](int, int, const float (&)[8]) {}, put);
       }
-      G::end_simd(r);
-      c.rem = true; c.first = false;
-      for (int i = nfull; i < nb; i++) {
-        Fr<IN> x; Fr<OUT> y;
-        for (int k = 0; k < IN; k++) x.v[k] = irow[(size_t)k * a.in_stride + i];
-        c.i = i;
-        G::template step<false>(r, c, x, y);
-        for (int k = 0; k < OUT; k++) emit(k, t0 + i, y.v[k]);
-      }
+      Saver s{a.state, a.V, v, 0u};
+      G::save(r, s);
     }
-    Saver s{a.state, a.V, v, 0u};
-    G::save(r, s);
+    if (mode & 2)
+      for (size_t e = 0; e < (size_t)OUT * a.n; e++) a.partial[(size_t)b * OUT * a.n + e] = cta_half_row_sum<NT>(&tile[e * NT], 0) + cta_half_row_sum<NT>(&tile[e * NT], 1);
   }
   if ((mode & 2) && a.ticket) {   // the fused finish of short launches (bank_kernel.cuh): CTA-order left fold into the mix
     for (uint32_t ch = 0; ch < (uint32_t)OUT; ch++)
       for (uint32_t t = 0; t < a.n; t++) {
-        float s = a.partial[(size_t)ch * a.n + t];
-        for (uint32_t q = 1; q < grid; q++) s += a.partial[((size_t)q * OUT + ch) * a.n + t];
+        const float s = cta_order_fold(a.partial + (size_t)ch * a.n + t, (size_t)OUT * a.n, grid, [](const float* p) { return *p; });
         float* p = a.mix + (size_t)ch * a.mix_stride + a.mix_offset + t;
         *p = a.mix_accumulate ? *p + s : s;
       }

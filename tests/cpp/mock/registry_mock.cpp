@@ -14,6 +14,7 @@
 
 #include "host/registry.h"
 #include "dsp/fdn_args.h"
+#include "dsp/mix_order.h"
 
 namespace fdsp {
 namespace host {
@@ -72,8 +73,7 @@ const char* registry_key(int) { return ""; }
 cudaError_t launch_mix_reduce(const float* partial, uint32_t nparts, uint32_t outs, uint32_t n, float* mix, uint32_t mix_stride, uint32_t mix_offset, int accumulate, cudaStream_t) {
   for (uint32_t c = 0; c < outs; c++)
     for (uint32_t t = 0; t < n; t++) {   // mix_reduce_kernel: CTA-order left fold
-      float s = partial[(size_t)c * n + t];
-      for (uint32_t b = 1; b < nparts; b++) s += partial[((size_t)b * outs + c) * n + t];
+      const float s = cta_order_fold(partial + (size_t)c * n + t, (size_t)outs * n, nparts, [](const float* q) { return *q; });
       float* p = mix + (size_t)c * mix_stride + mix_offset + t;
       *p = accumulate ? *p + s : s;
     }
@@ -87,11 +87,8 @@ cudaError_t launch_tree_mix(const float* rows, uint32_t V, uint32_t outs, uint32
       float x;
       if (pairwise) {
         float st[32];
-        for (uint32_t v = 0; v < V; v++) { float y = p[(size_t)v * vstep]; uint32_t q = v; int lvl = 0; while (q & 1u) { y = st[lvl] + y; q >>= 1; lvl++; } st[lvl] = y; }
-        int lvl = 0; uint32_t q = V;
-        while (!(q & 1u)) { q >>= 1; lvl++; }
-        x = st[lvl]; q >>= 1; lvl++;
-        for (; q; q >>= 1, lvl++) if (q & 1u) x = st[lvl] + x;
+        for (uint32_t v = 0; v < V; v++) carry_push(st, p[(size_t)v * vstep], v, 0);
+        x = carry_finish(st, V);
       } else { x = p[0]; for (uint32_t v = 1; v < V; v++) x += p[(size_t)v * vstep]; }
       mix[(size_t)ch * mix_stride + mix_offset + t] = x;
     }

@@ -1,5 +1,6 @@
 """CPU-only check of the DEVICE node templates: tests/cpp/device_emul.cpp compiles csrc/dsp/nodes.cuh for the host and runs one
-voice of a graph's fused program through bank_kernel's block structure; the output must equal the oracle's bit for bit.
+voice of a graph's fused program through the kernels' own block walk (csrc/dsp/voice_block.cuh walk_block); the output must equal the
+oracle's bit for bit.
 This is how device-side logic (here: the Dag form of nested Nets, and a sample of ordinary graphs) is exercised without a GPU.
 The GPU tests remain the parity tests proper; nothing here is part of the product."""
 import os

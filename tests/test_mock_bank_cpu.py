@@ -3,9 +3,10 @@ path, settings on a live bank, sequencer clock / edit / push / growth in place, 
 
 tests/cpp/mock/ builds the host sources against a stand-in <cuda_runtime.h> ("device" memory is host memory, calls are synchronous) and
 replaces the kernels by the device node library compiled for the CPU (FDSP_HOST_EMUL), one small shared object per graph class walking
-every voice through bank_kernel's per-thread block structure. The whole GPU test-suite then runs against that library in a subprocess
-(FDSP_B200_LIB selects it there and only there). What this does NOT cover is the CUDA side proper — the CTA mix tile, TMA table
-staging, the warp-per-voice FDN kernel itself (the mock runs the equivalent generic reverb program on its argument block, so the host side of
+every voice through the kernels' own block walk (csrc/dsp/voice_block.cuh) and summing the mix in the kernels' association
+(csrc/dsp/mix_order.h), so the per-CTA partials equal the GPU's bit for bit. The whole GPU test-suite then runs against that library in a
+subprocess (FDSP_B200_LIB selects it there and only there). What this does NOT cover is the CUDA side proper — the mix tile's shared
+memory and barriers, TMA table staging, the warp-per-voice FDN kernel itself (the mock runs the equivalent generic reverb program on its argument block, so the host side of
 the two-stage classes IS covered), stream concurrency — which the same tests check on a B200.
 The mock is test infrastructure: it is never built into, or loaded by, the product."""
 import hashlib

@@ -5,7 +5,7 @@ import sys
 import warnings
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-HDRS = ["math.cuh", "libm.cuh", "bank_args.h", "nodes.cuh", "bank_kernel.cuh"]   # = JITHDRS in csrc/Makefile
+HDRS = ["math.cuh", "libm.cuh", "bank_args.h", "nodes.cuh", "mix_order.h", "voice_block.cuh", "bank_kernel.cuh"]   # = JITHDRS in csrc/Makefile
 
 
 def compile_sig(sig):
